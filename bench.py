@@ -21,6 +21,12 @@ CPU algorithm on a bounded sample, timed on this box's host cores.
 `--impl reference`: times the reference's own CPU implementation (the oracle
 port, as-is semantics incl. the per-row Python pivot loop of util.py:86-90) on
 rank 0. The Python reference cannot travel to the GPU box; see DESIGN.md.
+
+`--dump-outputs DIR`: after the timed steps, rank 0 writes the results of the
+last timed step as DIR/<name>.npy (float32 / float64), so that two builds run
+with the same arguments (hence the same seeded inputs) can be compared output
+for output. Outputs larger than 64 MB in all are written for a fixed, seeded
+sample of the scenes (the same scenes in every array).
 """
 import argparse
 import json
@@ -122,6 +128,27 @@ class ClockSampler:
         reasons = sorted({names[i] for s in self.samples for i in range(4) if s[2 + i].lower().startswith("active")})
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": reasons, "samples": len(sm)}
+
+
+DUMP_BYTES = 60 * 10 ** 6           # array data of --dump-outputs; leaves room for the .npy headers under 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Writes `arrays` (name -> tensor with the scene index first, or None) as path/<name>.npy. Integer outputs
+    become float64 (exact). When every scene does not fit in DUMP_BYTES, all arrays keep the same scenes: a sorted
+    sample drawn with a fixed seed."""
+    import numpy as np
+    arrays = {k: v.detach() for k, v in arrays.items() if v is not None}
+    arrays = {k: (v if v.dtype in (torch.float32, torch.float64) else v.double()) for k, v in arrays.items()}
+    B = next(iter(arrays.values())).shape[0]
+    per_scene = sum(v[0].numel() * v.element_size() for v in arrays.values())
+    k = min(B, DUMP_BYTES // per_scene)
+    idx = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:k].sort().values if k < B else None
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        v = v.cpu() if idx is None else v.index_select(0, idx.to(v.device)).cpu()
+        np.save(os.path.join(path, name + ".npy"), v.numpy())
+    print("bench: wrote %d arrays of %d of %d scenes to %s" % (len(arrays), k, B, path), file=sys.stderr, flush=True)
 
 
 WORKLOAD = ("LCPFunction fwd+bwd (all 7 gradients), batch=%d scenes/GPU x 64 contacts x 2 fric dirs "
@@ -317,6 +344,8 @@ def run_world(args, rank, world, local_rank):
     e1.record()
     torch.cuda.synchronize()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"p": w_.p, "v": w_.v, "t": w_.t, "contacts": w_.counts})
     ms = e0.elapsed_time(e1)
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:
@@ -428,6 +457,8 @@ def run_cfg4(args, rank, world, local_rank):
     e1.record()
     torch.cuda.synchronize()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"p": w_.p, "v": w_.v, "t": w_.t, "contacts": w_.counts})
     ms = e0.elapsed_time(e1)
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:
@@ -642,6 +673,12 @@ def run_b200(args, rank, world, local_rank):
     ev[1].record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        names = ("zhat", None, "lam", "slack", "status", "iters", "resid")
+        outs = {n: t for n, t in zip(names, fo) if n}
+        if with_bwd:
+            outs.update(zip(("grad_Q", "grad_p", "grad_G", "grad_h", "grad_A", "grad_b", "grad_F"), bo))
+        dump_outputs(args.dump_outputs, outs)
     ms_total = ev[0].elapsed_time(ev[1])
     t = torch.tensor([ms_total], device=dev, dtype=torch.float64)
     if world > 1:
@@ -808,9 +845,15 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=128)
     ap.add_argument("--ref-batch", type=int, default=256)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step to DIR/<name>.npy (--impl b200)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 20 if args.config == "cfg4" and args.impl == "b200" else 5
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,8 +1,12 @@
-"""bench.py contract pieces that run without a GPU: the reference arm's JSON line and the helpers."""
+"""bench.py contract pieces: the reference arm's JSON line and the helpers (CPU), --dump-outputs (CPU and GPU)."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
+import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -56,3 +60,44 @@ def test_world_reference_arm_and_scene_generators():
     # neighbours of the hexagonal pile are closer than eps = 0.1: in contact before the first step
     d01 = (ic4["pos"][0, 1] - ic4["pos"][0, 2]).norm() - 20.0
     assert 0.0 < float(d01) < 0.1
+
+
+def test_dump_outputs_keeps_one_seeded_sample_of_scenes_under_64_mb(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    B = 4096
+    big = torch.randn(B, 64, 64, dtype=torch.float64)          # 32 KB per scene, 134 MB in all
+    scene = torch.arange(B, dtype=torch.int32)
+    bench.dump_outputs(str(tmp_path / "a"), {"big": big, "scene": scene, "absent": None})
+    bench.dump_outputs(str(tmp_path / "b"), {"big": big, "scene": scene})
+    assert sorted(os.listdir(tmp_path / "a")) == ["big.npy", "scene.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 64 * 10 ** 6
+    kept = np.load(tmp_path / "a" / "scene.npy")
+    assert kept.dtype == np.float64 and 0 < len(kept) < B and (np.diff(kept) > 0).all()
+    assert np.array_equal(np.load(tmp_path / "a" / "big.npy"), big[torch.from_numpy(kept).long()].numpy())
+    assert np.array_equal(np.load(tmp_path / "b" / "scene.npy"), kept)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_step(tmp_path):
+    """--dump-outputs writes every result of the timed path; at 64 scenes all of them, in the run's dtype."""
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--batch", "64", "--steps", "2", "--warmup", "1",
+                          "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    d = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][0])
+    assert d["steps"] == 2 and d["gpu_launches"] == 8
+    shapes = {"zhat": (64, 96), "lam": (64, 256), "slack": (64, 256), "status": (64,), "iters": (64,), "resid": (64,),
+              "grad_Q": (64, 96, 96), "grad_p": (64, 96), "grad_G": (64, 256, 96), "grad_h": (64, 256),
+              "grad_F": (64, 256, 256)}
+    assert sorted(os.listdir(tmp_path)) == sorted(k + ".npy" for k in shapes)
+    z = {k: np.load(tmp_path / (k + ".npy")) for k in shapes}
+    for k, s in shapes.items():
+        assert z[k].shape == s and z[k].dtype == (np.float64 if k in ("status", "iters") else np.float32), k
+    sys.path.insert(0, ROOT)
+    from lcp_physics_b200 import solve_forward
+    from lcp_physics_b200.scenes import make_scenes
+    inp = make_scenes(64, 32, 64, fd=2, e=0, dtype=torch.float32, seed=1000)
+    zhat = solve_forward(*(t.cuda() for t in inp), max_iter=10)[0].cpu().double()
+    err = (torch.from_numpy(z["zhat"]).double() - zhat).norm(dim=1) / zhat.norm(dim=1)
+    assert float(err.max()) < 1e-5
