@@ -156,6 +156,35 @@ int lcpb200_backward_host(lcpb200_handle_t h, int B,
 int lcpb200_find_contacts(int dtype, int B, int nb, int cap, double eps, const void* pos, const void* rad,
                           int32_t* body1, int32_t* body2, int32_t* counts, void* stream);
 
+/* lcpb200_find_contacts with pairs that never produce a contact (bodies.py:104-106 `add_no_contact`,
+ * contacts.py:60-61): skip is a bitmask over the lexicographic pair index q of (i < j), q = i (2 nb - i - 1) / 2 +
+ * j - i - 1, bit q & 31 of word q >> 5 (ceil(nb (nb - 1) / 64) words, shared by the batch). A skipped pair is
+ * neither counted nor listed; the order of the others is unchanged. skip == NULL is lcpb200_find_contacts. */
+int lcpb200_find_contacts_masked(int dtype, int B, int nb, int cap, double eps, const void* pos, const void* rad,
+                                 const uint32_t* skip, int32_t* body1, int32_t* body2, int32_t* counts, void* stream);
+
+/* Equality rows of joints (World.Je(), physics/world.py:156-170, Jacobians of physics/constraints.py) for B
+ * scenes with one constraint topology. Device pointers:
+ *   rows[e,4] int32        one {kind, body1, body2 or -1, aux} per row: kind 0 = unit row on dof aux of body1
+ *                          (X / Y / Rot / TotalConstraint), 1 / 2 = first / second row of a revolute Joint
+ *                          (J1 = [-y1, 1, 0] / [x1, 0, 1], J2 = [y2, -1, 0] / [-x2, 0, -1]) with pos1 = the lever
+ *                          of revolute joint aux (aux = -1: pos1 = 0, the FixedJoint's), 3 = [1,0,0] / [-1,0,0]
+ *                          (the FixedJoint's rotation row); pos2 = p_body1 + pos1 - p_body2
+ *   pos[B,nb,2]            body centres;  pos1[B,nj,2]: levers of the nj revolute joints (NULL if nj == 0)
+ *   A[B,e,3nb]             OUT: dense rows, every element written
+ *   v[B,3nb], ge[B,e]      optional (both or neither): ge = A v, the b of post-stabilisation (engines.py:87)
+ * e <= 256. */
+int lcpb200_joint_rows(int dtype, int B, int nb, int e, int nj, const int32_t* rows, const void* pos,
+                       const void* pos1, const void* v, void* A, void* ge, void* stream);
+
+/* Joint.move (constraints.py:38-45) of the nj revolute joints of B scenes:
+ *   rot1[s,k] = rot1_start[s,k] + v[s, 3 joint_body[k]] dts[s],  pos1[s,k] = r1[s,k] (cos, sin)(rot1[s,k])
+ * joint_body[nj] int32 (body 1 of each joint), rot1_start / r1 / rot1 [B,nj], v[B,3nb], dts[B], pos1[B,nj,2].
+ * done[B] (uint8, may be NULL): scenes with done[s] != 0 keep rot1 and pos1. rot1_start may alias rot1. */
+int lcpb200_joint_move(int dtype, int B, int nb, int nj, const int32_t* joint_body, const void* rot1_start,
+                       const void* r1, const void* v, const void* dts, const uint8_t* done, void* rot1, void* pos1,
+                       void* stream);
+
 /* Geometry and material of the pairs selected by lcpb200_find_contacts (contacts.py:69-77, world.py:144-151,
  * :213-224), for callers that do not differentiate through the contact generation:
  *   normal[B,cap,2] = (pos1 - pos2) / dist, penetration[B,cap] = r1 + r2 - dist (-1e30 in unused slots),

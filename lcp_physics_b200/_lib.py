@@ -37,6 +37,9 @@ _SIGS = {
     "lcpb200_engine_backward": (ctypes.c_int, [_vp] + [ctypes.c_int] * 4 + [ctypes.c_double] + [_vp] * 29 +
                                 [ctypes.c_uint, _vp]),
     "lcpb200_find_contacts": (ctypes.c_int, [ctypes.c_int] * 4 + [ctypes.c_double] + [_vp] * 6),
+    "lcpb200_find_contacts_masked": (ctypes.c_int, [ctypes.c_int] * 4 + [ctypes.c_double] + [_vp] * 7),
+    "lcpb200_joint_rows": (ctypes.c_int, [ctypes.c_int] * 5 + [_vp] * 7),
+    "lcpb200_joint_move": (ctypes.c_int, [ctypes.c_int] * 4 + [_vp] * 9),
     "lcpb200_contact_geometry": (ctypes.c_int, [ctypes.c_int] * 4 + [_vp] * 14),
     "lcpb200_assemble": (ctypes.c_int, [ctypes.c_int] * 4 + [ctypes.c_double] + [_vp] * 17),
     "lcpb200_assemble_backward": (ctypes.c_int, [ctypes.c_int] * 4 + [ctypes.c_double] + [_vp] * 25),

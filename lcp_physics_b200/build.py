@@ -26,7 +26,7 @@ NVCC_FLAGS = [
 DUAL_DEPS = ["lcp_kernels.cu", "lcp_launch.h", "lcp_device.cuh", "lcp_lu.cuh", "lcp_solver.cuh"]
 COND_DEPS = ["lcp_cond_kernels.cu", "lcp_cond_launch.h", "lcp_device.cuh", "lcp_condensed.cuh"]
 BAND_DEPS = ["lcp_band_kernels.cu", "lcp_band_launch.h", "lcp_device.cuh", "lcp_condensed.cuh", "lcp_banded.cuh"]
-API_DEPS = ["lcpb200.cu", "lcp_assemble.cuh", "lcp_contacts.cuh", "../../include/lcpb200.h"] + DUAL_DEPS[1:] + COND_DEPS[1:] + BAND_DEPS[1:]
+API_DEPS = ["lcpb200.cu", "lcp_assemble.cuh", "lcp_contacts.cuh", "lcp_joints.cuh", "../../include/lcpb200.h"] + DUAL_DEPS[1:] + COND_DEPS[1:] + BAND_DEPS[1:]
 
 # dual-form kernels: one TU per (dtype, residency mode); condensed kernels: one per (dtype, NS)
 DUAL_VARIANTS = [(t, m) for t in ("float", "double") for m in (0, 1, 2)]

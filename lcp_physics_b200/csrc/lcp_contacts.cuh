@@ -9,7 +9,9 @@
 // the LCP the engine builds -- and compacts the touching pairs IN THAT ORDER with a block-wide exclusive scan
 // (ballot prefix inside a warp, warp totals through shared memory): deterministic, no atomics, no sort.
 // Outputs: the pair list body1 / body2 [B, cap] (padded with the pair (0, 1)), and the TRUE number of touching
-// pairs per scene (which may exceed cap: the caller checks). The contact geometry (normal, p1, p2, penetration)
+// pairs per scene (which may exceed cap: the caller checks). An optional skip bitmask over the pair index q (bit
+// q & 31 of word q >> 5, shared by the batch) removes pairs that never produce a contact (`add_no_contact`,
+// bodies.py:104-106, contacts.py:60-61): a skipped pair is neither counted nor listed. The contact geometry (normal, p1, p2, penetration)
 // is evaluated by the caller on the selected pairs only (O(cap), differentiable in torch), so this kernel
 // replaces the O(nb^2) part: at nb = 513 it tests 131 328 pairs per scene.
 #pragma once
@@ -27,8 +29,9 @@ __device__ __forceinline__ long long pairs_before(long long i, long long nb) { r
 
 template <typename T>
 __global__ void __launch_bounds__(NT) find_contacts_kernel(int B, int nb, int cap, T eps, const T* __restrict__ pos,
-                                                           const T* __restrict__ rad, int32_t* __restrict__ body1,
-                                                           int32_t* __restrict__ body2, int32_t* __restrict__ counts) {
+                                                           const T* __restrict__ rad, const uint32_t* __restrict__ skip,
+                                                           int32_t* __restrict__ body1, int32_t* __restrict__ body2,
+                                                           int32_t* __restrict__ counts) {
   __shared__ int warp_tot[NT / 32];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const long long npairs = (long long)nb * (nb - 1) / 2;
@@ -57,10 +60,13 @@ __global__ void __launch_bounds__(NT) find_contacts_kernel(int B, int nb, int ca
       for (int u = 0; u < ITEMS; ++u) {
         pi[u] = i; pj[u] = j;
         if (q + u < npairs) {
-          const T dx = P[2 * i] - P[2 * j], dy = P[2 * i + 1] - P[2 * j + 1];
-          const T dist = sqrt(dx * dx + dy * dy);
-          const T pen = R[i] + R[j] - dist;                      // contacts.py:70-73
-          if (!(pen < -eps)) hit |= 1u << u;                     // `if penetration < -eps: return`
+          const long long qu = q + u;
+          if (skip == nullptr || !((skip[qu >> 5] >> (qu & 31)) & 1u)) {   // `if geom1 in geom2.no_contact: return`
+            const T dx = P[2 * i] - P[2 * j], dy = P[2 * i + 1] - P[2 * j + 1];
+            const T dist = sqrt(dx * dx + dy * dy);
+            const T pen = R[i] + R[j] - dist;                    // contacts.py:70-73
+            if (!(pen < -eps)) hit |= 1u << u;                   // `if penetration < -eps: return`
+          }
           if (++j == nb) { ++i; j = i + 1; }
         }
       }
@@ -130,10 +136,10 @@ static void launch_contact_geometry(int B, int nb, int cap, const T* pos, const 
 }
 
 template <typename T>
-static void launch_find_contacts(int B, int nb, int cap, T eps, const T* pos, const T* rad, int32_t* body1,
-                                 int32_t* body2, int32_t* counts, int num_sms, cudaStream_t st) {
+static void launch_find_contacts(int B, int nb, int cap, T eps, const T* pos, const T* rad, const uint32_t* skip,
+                                 int32_t* body1, int32_t* body2, int32_t* counts, int num_sms, cudaStream_t st) {
   const int grid = B < 8 * num_sms ? B : 8 * num_sms;
-  find_contacts_kernel<T><<<grid, NT, 0, st>>>(B, nb, cap, eps, pos, rad, body1, body2, counts);
+  find_contacts_kernel<T><<<grid, NT, 0, st>>>(B, nb, cap, eps, pos, rad, skip, body1, body2, counts);
 }
 
 }  // namespace cts

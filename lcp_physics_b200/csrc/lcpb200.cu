@@ -13,6 +13,7 @@
 #include "lcp_cond_launch.h"
 #include "lcp_band_launch.h"
 #include "lcp_contacts.cuh"
+#include "lcp_joints.cuh"
 
 using namespace lcpb200;
 using cnd::CPlan;
@@ -897,8 +898,9 @@ extern "C" int lcpb200_engine_backward(lcpb200_handle_t h, int B, int nb, int nc
 }
 
 // ------------------------------------------------------------------ assembly
-extern "C" int lcpb200_find_contacts(int dtype, int B, int nb, int cap, double eps, const void* pos, const void* rad,
-                                     int32_t* body1, int32_t* body2, int32_t* counts, void* stream) {
+extern "C" int lcpb200_find_contacts_masked(int dtype, int B, int nb, int cap, double eps, const void* pos,
+                                            const void* rad, const uint32_t* skip, int32_t* body1, int32_t* body2,
+                                            int32_t* counts, void* stream) {
   if (dtype != LCPB200_F32 && dtype != LCPB200_F64) return fail("bad dtype");
   if (B < 0 || nb <= 0 || cap <= 0) return fail("find_contacts: need B >= 0, nb > 0, cap > 0");
   if (!pos || !rad || !body1 || !body2 || !counts) return fail("find_contacts: NULL argument");
@@ -908,9 +910,59 @@ extern "C" int lcpb200_find_contacts(int dtype, int B, int nb, int cap, double e
   CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   cudaStream_t st = (cudaStream_t)stream;
   if (dtype == LCPB200_F32)
-    cts::launch_find_contacts<float>(B, nb, cap, (float)eps, (const float*)pos, (const float*)rad, body1, body2, counts, sms, st);
+    cts::launch_find_contacts<float>(B, nb, cap, (float)eps, (const float*)pos, (const float*)rad, skip, body1, body2,
+                                     counts, sms, st);
   else
-    cts::launch_find_contacts<double>(B, nb, cap, eps, (const double*)pos, (const double*)rad, body1, body2, counts, sms, st);
+    cts::launch_find_contacts<double>(B, nb, cap, eps, (const double*)pos, (const double*)rad, skip, body1, body2,
+                                      counts, sms, st);
+  CK(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int lcpb200_find_contacts(int dtype, int B, int nb, int cap, double eps, const void* pos, const void* rad,
+                                     int32_t* body1, int32_t* body2, int32_t* counts, void* stream) {
+  return lcpb200_find_contacts_masked(dtype, B, nb, cap, eps, pos, rad, nullptr, body1, body2, counts, stream);
+}
+
+extern "C" int lcpb200_joint_rows(int dtype, int B, int nb, int e, int nj, const int32_t* rows, const void* pos,
+                                  const void* pos1, const void* v, void* A, void* ge, void* stream) {
+  if (dtype != LCPB200_F32 && dtype != LCPB200_F64) return fail("bad dtype");
+  if (B < 0 || nb <= 0 || e <= 0 || nj < 0) return fail("joint_rows: need B >= 0, nb > 0, e > 0, nj >= 0");
+  if (e > jnt::MAX_ROWS) return fail("joint_rows: more than " + std::to_string(jnt::MAX_ROWS) + " rows");
+  if (!rows || !pos || !A || (nj > 0 && !pos1)) return fail("joint_rows: NULL argument");
+  if (ge && !v) return fail("joint_rows: ge needs v");
+  if (B == 0) return 0;
+  int dev = 0, sms = 0;
+  CK(cudaGetDevice(&dev));
+  CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == LCPB200_F32)
+    jnt::launch_joint_rows<float>(B, nb, e, nj, rows, (const float*)pos, (const float*)pos1, (const float*)v, (float*)A,
+                                  (float*)ge, sms, st);
+  else
+    jnt::launch_joint_rows<double>(B, nb, e, nj, rows, (const double*)pos, (const double*)pos1, (const double*)v,
+                                   (double*)A, (double*)ge, sms, st);
+  CK(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int lcpb200_joint_move(int dtype, int B, int nb, int nj, const int32_t* joint_body, const void* rot1_start,
+                                  const void* r1, const void* v, const void* dts, const uint8_t* done, void* rot1,
+                                  void* pos1, void* stream) {
+  if (dtype != LCPB200_F32 && dtype != LCPB200_F64) return fail("bad dtype");
+  if (B < 0 || nb <= 0 || nj < 0) return fail("joint_move: need B >= 0, nb > 0, nj >= 0");
+  if (B == 0 || nj == 0) return 0;
+  if (!joint_body || !rot1_start || !r1 || !v || !dts || !rot1 || !pos1) return fail("joint_move: NULL argument");
+  int dev = 0, sms = 0;
+  CK(cudaGetDevice(&dev));
+  CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == LCPB200_F32)
+    jnt::launch_joint_move<float>(B, nb, nj, joint_body, (const float*)rot1_start, (const float*)r1, (const float*)v,
+                                  (const float*)dts, done, (float*)rot1, (float*)pos1, sms, st);
+  else
+    jnt::launch_joint_move<double>(B, nb, nj, joint_body, (const double*)rot1_start, (const double*)r1,
+                                   (const double*)v, (const double*)dts, done, (double*)rot1, (double*)pos1, sms, st);
   CK(cudaGetLastError());
   return 0;
 }

@@ -229,3 +229,58 @@ def make_ball_pile(B, nballs=512, cols=32, seed=0, dtype=torch.float64, r=10.0, 
     fric = torch.full((B, nb), 0.9, dtype=f64)               # utils.py:22-24 defaults
     rest = torch.full((B, nb), 0.5, dtype=f64)
     return {k_: t.to(dtype) for k_, t in dict(pos=pos, vel=vel, rad=rad, mass=mass, fric=fric, rest=rest).items()}
+
+
+JOINT_CHAIN_LINKS = 5
+
+
+def make_joint_chain(B, seed=0, dtype=torch.float64, links=JOINT_CHAIN_LINKS):
+    """Initial conditions of B jointed `BatchedWorld` scenes (the circle analogue of the reference's chain_demo,
+    demos/demo.py:62-90): body 0 a huge pinned ball that plays the floor (radius 2000), bodies 1..links a chain of
+    overlapping circles (radius 15, 25 apart) hung from a world Joint, each link jointed to the one above it at their
+    midpoint (Joint(k + 1, k, ...), i1 > i2 as in chain_demo), then a ball thrown at the chain, a ball held by X and
+    Rot constraints falling onto the floor, and a FixedJoint pair falling onto the floor. Each scene has its own
+    velocities, masses, friction, restitution and anchor jitter. Returns a dict of [B, ...] tensors; `anchor`
+    [B, links, 2] are the joint anchors (joint_chain_specs turns them into constraint specs)."""
+    g = torch.Generator().manual_seed(seed)
+    L = links
+    nb = L + 5
+    u = lambda *s: torch.rand(B, *s, generator=g, dtype=torch.float64)
+    pos = torch.zeros(B, nb, 2, dtype=torch.float64)
+    rad = torch.full((B, nb), 15.0, dtype=torch.float64)
+    pos[:, 0] = torch.tensor([300.0, 2500.0])
+    rad[:, 0] = 2000.0
+    for k in range(L):
+        pos[:, 1 + k] = torch.tensor([300.0, 130.0 + 25.0 * k])
+    anchor = torch.stack([torch.tensor([300.0, 105.0 + 25.0 * k]) for k in range(L)]).expand(B, L, 2) \
+        + (u(L, 2) - 0.5)
+    pos[:, L + 1] = torch.tensor([180.0, 190.0])                                      # striker
+    pos[:, L + 2] = torch.tensor([470.0, 440.0])                                      # X + Rot constrained
+    rad[:, L + 2] = 20.0
+    pos[:, L + 3] = torch.tensor([120.0, 455.0])                                      # FixedJoint pair
+    pos[:, L + 4] = torch.tensor([155.0, 455.0])
+    vel = torch.zeros(B, nb, 3, dtype=torch.float64)
+    vel[:, 1:L + 1, 1] = (u(L) - 0.5) * 4.0
+    vel[:, L + 1] = torch.stack([(u() - 0.5) * 0.4, 140.0 + 20.0 * u(), -30.0 - 10.0 * u()], 1)
+    vel[:, L + 2, 2] = 40.0 + 10.0 * u()
+    vel[:, L + 3:, 2] = (30.0 + 10.0 * u()).unsqueeze(1)
+    vel[:, L + 3:, 1] = ((u() - 0.5) * 10.0).unsqueeze(1)
+    mass = 0.5 + u(nb)
+    mass[:, 0] = 1.0
+    fric = 0.2 + 0.7 * u(nb)
+    rest = 0.2 + 0.5 * u(nb)
+    out = dict(pos=pos, vel=vel, rad=rad, mass=mass, fric=fric, rest=rest, anchor=anchor)
+    return {k_: t.to(dtype) for k_, t in out.items()}
+
+
+def joint_chain_specs(anchor, joints=True):
+    """(joints, no_contact) of make_joint_chain's scene for anchor [B, links, 2] (BatchedWorld) or [links, 2] (one
+    world). joints=False: no joints or constraints (the pins only), the same no-contact pairs."""
+    from .constraints import FixedJoint, Joint, RotConstraint, XConstraint
+    L = anchor.shape[-2]
+    if not joints:
+        return [], [(k, k + 1) for k in range(1, L)]
+    js = [Joint(1, None, anchor[..., 0, :])]
+    js += [Joint(k + 1, k, anchor[..., k, :]) for k in range(1, L)]
+    js += [XConstraint(L + 2), RotConstraint(L + 2), FixedJoint(L + 3, L + 4)]
+    return js, [(k, k + 1) for k in range(1, L)]
